@@ -10,6 +10,10 @@ A "step" = one forward + backward pass of the public API (`LightplaneRenderer` m
 a random target image) over the whole ray batch; at N>1 every rank renders its own FullHD batch
 (weak scaling) and the grid / MLP gradients are SUM-all-reduced over NCCL inside the step.
 Prints ONE JSON line on rank 0.  See DESIGN.md "Measurement" for how every field is derived.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (rendered features, loss, and the
+gradient of every trained tensor) as DIR/<name>.npy in float32.  The inputs depend only on the arguments (fixed
+seeds), so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -85,6 +89,28 @@ def camera_rays(width, height, seed, device, fov=0.62, clip_to_volume=False):
         far = torch.full((n,), 2.6 + 1.75)
     grid_idx = torch.zeros(n, dtype=torch.int32)
     return dirs, origins, grid_idx, near, far
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """Write every array as `outdir/<name>.npy` in float32, at most DUMP_BYTES in all.  Smallest first, an array larger
+    than an equal share of what is left keeps a sample of its rows (first axis) drawn with a fixed seed, so the sample
+    depends only on the array's shape."""
+    import numpy as np
+
+    os.makedirs(outdir, exist_ok=True)
+    budget, left = DUMP_BYTES - (1 << 20), len(arrays)  # 1 MB for the .npy headers
+    for name, v in sorted(arrays.items(), key=lambda kv: kv[1].numel()):
+        v = v.detach().float().cpu()
+        share = budget // left
+        if v.numel() * 4 > share:
+            rows = max(1, share // (v[0].numel() * 4))
+            v = v[torch.randperm(v.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+        np.save(os.path.join(outdir, name + ".npy"), v.numpy())
+        budget -= v.numel() * 4
+        left -= 1
 
 
 def workload_stats(rays_t, width, samples, plane, tile_walk, device):
@@ -297,7 +323,12 @@ def main():
     ap.add_argument("--samples", type=int, default=None)
     ap.add_argument("--plane", type=int, default=None)
     ap.add_argument("--grid-chn", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's features, loss and gradients as DIR/<name>.npy (float32, at most "
+                         "64 MB: larger outputs keep a fixed seeded sample of their rows)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repository's CUDA path (--impl ours)")
     cfg5 = args.workload == "cfg5"
     globals().update(S=args.samples or (256 if cfg5 else S), PLANE=args.plane or (128 if cfg5 else PLANE),
                      C=args.grid_chn or (32 if cfg5 else C))
@@ -437,12 +468,28 @@ def main():
         e2e_step()
     e2e_finish()
 
+    last = {}
+
+    def timed_step():
+        feat, loss = step(resident, target)
+        last["features"], last["loss"] = feat.detach(), loss.detach()
+
     sampler = ClockSampler(local_rank) if rank == 0 else None
     comm_events.clear()
     _cabi.profile_begin()
-    ms = timed(lambda: step(resident, target), args.steps)
-    launches = _cabi.profile_end()
-    clocks = sampler.stop() if sampler else None
+    try:
+        ms = timed(timed_step, args.steps)
+        launches = _cabi.profile_end()
+    finally:  # nvidia-smi must not outlive a failed step
+        clocks = sampler.stop() if sampler else None
+    # taken before the later timed regions, which run the step again and overwrite the gradients
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = {"features": last["features"], "loss": last["loss"], "grad_grid": grids[0].grad}
+        outputs.update({"grad_" + k.replace(".", "_"): p.grad for k, p in model.named_parameters()})
+        if cfg5:
+            outputs["grad_splat_features"] = splat_feat.grad
+        outputs = {k: v.cpu() for k, v in outputs.items()}
     comm_ms = sum(a.elapsed_time(b) for a, b in comm_events) / max(len(comm_events), 1) if comm_events else 0.0
     ms_e2e = timed(e2e_step, args.steps, e2e_finish)
 
@@ -557,6 +604,8 @@ def main():
                 line["gpu_comparator"] = {r["workload"].split(" rays")[0]: r.get("reference_triton", {}).get("rays_per_s") for r in rows}
             except Exception:
                 pass
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
