@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define LP_ABI_VERSION 2
+#define LP_ABI_VERSION 3
 #define LP_MAX_GRIDS 8   /* grids per grid-list */
 #define LP_MAX_LAYERS 8  /* layers per MLP */
 
@@ -136,6 +136,23 @@ int lp_render_backward(void* stream, const lp_march_cfg* cfg, const lp_decoder_s
                        const float* grad_neg_log_transmittance, const float* grad_features,
                        int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
                        float* grad_mlp_params, float* grad_encoding);
+
+/* Renderer backward with gradients w.r.t. the ray geometry (an extension; the reference has no
+ * such gradients).  Arguments and outputs of lp_render_backward, plus
+ *   grad_origins [N,3], grad_directions [N,3]: fully written; either may be NULL (not wanted).
+ * With a sample at p_j = o + t_j d read at x_j = c(p_j) (c = the contraction or the identity) and
+ * a_j the gradient w.r.t. its sampled feature row, g_j = sum_grids sum_taps <v_t, a_j> grad w_t(x_j),
+ * dL/do = sum_j J_c(p_j)^T g_j and dL/dd = sum_j t_j J_c(p_j)^T g_j.  The OOB mask, scaffold and
+ * noise are piecewise constant in position and add no terms; near / far get no gradient. */
+int lp_render_backward_rays(void* stream, const lp_march_cfg* cfg, const lp_decoder_spec* spec,
+                            const lp_rays* rays, const lp_grid_list* grid,
+                            const lp_grid_list* color_grid, const lp_grid_list* scaffold,
+                            const float* mlp_params, const float* ray_length, const float* features,
+                            int32_t features_stride, const float* grad_ray_length,
+                            const float* grad_neg_log_transmittance, const float* grad_features,
+                            int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
+                            float* grad_mlp_params, float* grad_encoding, float* grad_origins,
+                            float* grad_directions);
 
 /* Splatter forward.  Replaces BOTH launches of `fw_kernel` (features, then unit weights),
  * lightplane_splatter.py:503-539 / splatter_fw.py:71-165, in one pass: accumulates

@@ -13,7 +13,7 @@ from typing import Optional, Sequence
 import torch
 
 LP_MAX_GRIDS = 8
-LP_ABI_VERSION = 2
+LP_ABI_VERSION = 3
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB_PATH = os.path.join(_HERE, "csrc", "liblightplane_b200.so")
@@ -96,6 +96,10 @@ _PROTOTYPES = {
     "lp_render_backward": (
         C.c_int,
         [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P, _P, _P],
+    ),
+    "lp_render_backward_rays": (
+        C.c_int,
+        [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P],
     ),
     "lp_splat_forward": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "lp_splat_backward": (C.c_int, [_P, _P, _P, _P, _P, _P]),

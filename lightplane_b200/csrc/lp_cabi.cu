@@ -305,13 +305,16 @@ int lp_render_forward(void* stream, const lp_march_cfg* cfg, const lp_decoder_sp
   return lp_check_launch("lp_render_forward");
 }
 
-int lp_render_backward(void* stream, const lp_march_cfg* cfg, const lp_decoder_spec* spec,
-                       const lp_rays* rays, const lp_grid_list* grid, const lp_grid_list* color_grid,
-                       const lp_grid_list* scaffold, const float* mlp_params, const float* ray_length,
-                       const float* features, int32_t features_stride, const float* grad_ray_length,
-                       const float* grad_neg_log_transmittance, const float* grad_features,
-                       int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
-                       float* grad_mlp_params, float* grad_encoding) {
+// lp_render_backward and lp_render_backward_rays: grad_origins / grad_directions NULL = that gradient is not wanted;
+// with both NULL the kernels without the ray-geometry terms run.
+static int lp_render_backward_impl(void* stream, const lp_march_cfg* cfg, const lp_decoder_spec* spec,
+                                   const lp_rays* rays, const lp_grid_list* grid, const lp_grid_list* color_grid,
+                                   const lp_grid_list* scaffold, const float* mlp_params, const float* ray_length,
+                                   const float* features, int32_t features_stride, const float* grad_ray_length,
+                                   const float* grad_neg_log_transmittance, const float* grad_features,
+                                   int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
+                                   float* grad_mlp_params, float* grad_encoding, float* grad_origins,
+                                   float* grad_directions) {
   LpRenderArgs a;
   int rc;
   if ((rc = lp_render_common(cfg, spec, rays, grid, color_grid, scaffold, mlp_params, &a))) return rc;
@@ -328,21 +331,24 @@ int lp_render_backward(void* stream, const lp_march_cfg* cfg, const lp_decoder_s
   io.g_len = grad_ray_length; io.g_nlt = grad_neg_log_transmittance; io.g_feat = grad_features;
   io.g_feat_stride = grad_features_stride;
   io.g_grid = grad_grid; io.g_cgrid = grad_color_grid; io.g_params = grad_mlp_params; io.g_enc = grad_encoding;
+  io.g_org = grad_origins; io.g_dir = grad_directions;
+  const bool rayg = grad_origins || grad_directions;
   const bool fast = !lp_only_generic();
   if (fast && lptc::lp_tc_render_supported(a)) {
-    if ((rc = lptc::lp_tc_render_backward(st, a, mlp_params, io))) LP_FAIL(rc, "fast backward launch setup failed");
+    if ((rc = lptc::lp_tc_render_backward(st, a, mlp_params, io, rayg))) LP_FAIL(rc, "fast backward launch setup failed");
     return lp_check_launch("lp_render_backward(fast)");
   }
-  if (fast && lptc::lp_cg_render_supported(a)) {
+  // the other tensor-core variants have no ray-geometry terms: such requests take the generic kernel
+  if (fast && !rayg && lptc::lp_cg_render_supported(a)) {
     if ((rc = lptc::lp_cg_render_backward(st, a, mlp_params, io))) LP_FAIL(rc, "colour-grid backward launch setup failed");
     return lp_check_launch("lp_render_backward(colour grid)");
   }
-  if (fast && lptc::lp_tcw_forward_supported(a)) {
+  if (fast && !rayg && lptc::lp_tcw_forward_supported(a)) {
     if ((rc = lptc::lp_tcw_render_backward(st, a, mlp_params, io))) LP_FAIL(rc, "hidden-64 backward launch setup failed");
     return lp_check_launch("lp_render_backward(hidden 64)");
   }
   lptc::DeepPlan dpl;
-  if (fast && lptc::lp_deep_plan(a, &dpl)) {
+  if (fast && !rayg && lptc::lp_deep_plan(a, &dpl)) {
     if ((rc = lptc::lp_deep_render_backward(st, a, dpl, mlp_params, io))) LP_FAIL(rc, "layer-count-general backward launch setup failed");
     return lp_check_launch("lp_render_backward(deep)");
   }
@@ -350,12 +356,45 @@ int lp_render_backward(void* stream, const lp_march_cfg* cfg, const lp_decoder_s
   const int per_warp = (a.A.total + 3 * a.D.max_dim + 2 * a.D.in_c + a.D.n_feat) * LP_LS;
   int warps, pin; size_t bytes;
   if ((rc = lp_plan_smem(pf, pf, per_warp, &warps, &pin, &bytes))) return rc;
-  if (LP_SET_SMEM(lp_render_bwd_generic_kernel, bytes)) LP_FAIL(LP_ERR_CUDA, "cannot raise dynamic smem limit");
   const int rays_per_block = warps * LP_WARP;
   dim3 gridDimv((a.R.n + rays_per_block - 1) / rays_per_block), block(rays_per_block);
-  LP_LAUNCH(lp_render_bwd_generic_kernel, gridDimv, block, bytes, st, a.R, a.M, a.D, a.A, a.G, a.CG, a.SC,
-            a.use_scaffold, mlp_params, pin, io);
+  if (rayg) {
+    if (LP_SET_SMEM(lp_render_bwd_generic_kernel<true>, bytes)) LP_FAIL(LP_ERR_CUDA, "cannot raise dynamic smem limit");
+    LP_LAUNCH(lp_render_bwd_generic_kernel<true>, gridDimv, block, bytes, st, a.R, a.M, a.D, a.A, a.G, a.CG, a.SC,
+              a.use_scaffold, mlp_params, pin, io);
+  } else {
+    if (LP_SET_SMEM(lp_render_bwd_generic_kernel<false>, bytes)) LP_FAIL(LP_ERR_CUDA, "cannot raise dynamic smem limit");
+    LP_LAUNCH(lp_render_bwd_generic_kernel<false>, gridDimv, block, bytes, st, a.R, a.M, a.D, a.A, a.G, a.CG, a.SC,
+              a.use_scaffold, mlp_params, pin, io);
+  }
   return lp_check_launch("lp_render_backward");
+}
+
+int lp_render_backward(void* stream, const lp_march_cfg* cfg, const lp_decoder_spec* spec,
+                       const lp_rays* rays, const lp_grid_list* grid, const lp_grid_list* color_grid,
+                       const lp_grid_list* scaffold, const float* mlp_params, const float* ray_length,
+                       const float* features, int32_t features_stride, const float* grad_ray_length,
+                       const float* grad_neg_log_transmittance, const float* grad_features,
+                       int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
+                       float* grad_mlp_params, float* grad_encoding) {
+  return lp_render_backward_impl(stream, cfg, spec, rays, grid, color_grid, scaffold, mlp_params, ray_length, features,
+                                 features_stride, grad_ray_length, grad_neg_log_transmittance, grad_features,
+                                 grad_features_stride, grad_grid, grad_color_grid, grad_mlp_params, grad_encoding,
+                                 nullptr, nullptr);
+}
+
+int lp_render_backward_rays(void* stream, const lp_march_cfg* cfg, const lp_decoder_spec* spec,
+                            const lp_rays* rays, const lp_grid_list* grid, const lp_grid_list* color_grid,
+                            const lp_grid_list* scaffold, const float* mlp_params, const float* ray_length,
+                            const float* features, int32_t features_stride, const float* grad_ray_length,
+                            const float* grad_neg_log_transmittance, const float* grad_features,
+                            int32_t grad_features_stride, float* grad_grid, float* grad_color_grid,
+                            float* grad_mlp_params, float* grad_encoding, float* grad_origins,
+                            float* grad_directions) {
+  return lp_render_backward_impl(stream, cfg, spec, rays, grid, color_grid, scaffold, mlp_params, ray_length, features,
+                                 features_stride, grad_ray_length, grad_neg_log_transmittance, grad_features,
+                                 grad_features_stride, grad_grid, grad_color_grid, grad_mlp_params, grad_encoding,
+                                 grad_origins, grad_directions);
 }
 
 // ---- plain splatter ---------------------------------------------------------------------------

@@ -1,5 +1,6 @@
 // Device-side building blocks shared by all kernels of the hot path: grid-list addressing
-// (tri/bi-linear taps), the depth schedule, coordinate contraction, activations and the hash RNG.
+// (tri/bi-linear taps), the depth schedule, coordinate contraction, activations, the hash RNG and the gradient w.r.t.
+// a sample's position.
 // Every function cites the reference lines whose semantics it implements
 // (paths relative to facebookresearch/lightplane).
 #pragma once
@@ -214,6 +215,102 @@ LP_DEVICE int lp_taps(const LpGrid& g, int C, int b, float x, float y, float z, 
     off[c] = bbase + ((long long)iv * U + iu) * C;
   }
   return 4;
+}
+
+// ---------------------------------------------------------------------------------------------
+// gradient w.r.t. the sample position (ray-geometry gradients of lp_render_backward_rays)
+// ---------------------------------------------------------------------------------------------
+// One axis of lp_axis / lp_corner with the derivative of both corner weights w.r.t. the coordinate: d frac / d p =
+// size / 2, 0 on pinned singleton axes; a corner outside the grid has weight and derivative 0 (zero padding).
+LP_DEVICE void lp_axis_d(float p, int size, float (&w)[2], float (&dw)[2], int (&idx)[2]) {
+  float i0, frac;
+  lp_axis(p, size, i0, frac);
+  const float s = size > 1 ? 0.5f * (float)size : 0.f;
+#pragma unroll
+  for (int hi = 0; hi < 2; ++hi) {
+    const float ia = i0 + (float)hi;
+    const bool ok = (ia >= 0.f) && (ia < (float)size);
+    w[hi] = ok ? (hi ? frac : 1.f - frac) : 0.f;
+    dw[hi] = ok ? (hi ? s : -s) : 0.f;
+    idx[hi] = (int)fminf(fmaxf(ia, 0.f), (float)(size - 1));
+  }
+}
+
+// Gradient w.r.t. the grid-space point (x,y,z) of sum over the grids of G and their taps t of w_t(x,y,z) <v_t, a>, i.e.
+// sum_t <v_t, a> grad w_t, for the sampled-feature gradient a of one sample.  `dot(row)` returns <row, a> for the C
+// floats of a texel row; it is called only for taps whose weight gradient is non-zero.  Adds into (gx, gy, gz).
+template <class Dot>
+LP_DEVICE void lp_pos_grad(const LpGridSet& G, int b, float x, float y, float z, const Dot& dot, float& gx, float& gy,
+                           float& gz) {
+  const int C = G.C;
+  for (int gi = 0; gi < G.n; ++gi) {
+    const LpGrid& g = G.g[gi];
+    if (g.kind == LP_VOXEL) {
+      float wx[2], dwx[2], wy[2], dwy[2], wz[2], dwz[2];
+      int ix[2], iy[2], iz[2];
+      lp_axis_d(x, g.W, wx, dwx, ix);
+      lp_axis_d(y, g.H, wy, dwy, iy);
+      lp_axis_d(z, g.D, wz, dwz, iz);
+      const long long bbase = g.base + (long long)b * g.D * g.H * g.W * C;
+#pragma unroll
+      for (int c = 0; c < 8; ++c) {
+        const int i = c & 1, j = (c >> 1) & 1, k = c >> 2;
+        const float ex = dwx[i] * wy[j] * wz[k], ey = wx[i] * dwy[j] * wz[k], ez = wx[i] * wy[j] * dwz[k];
+        if (ex != 0.f || ey != 0.f || ez != 0.f) {
+          const float d = dot(G.data + bbase + ((long long)(iz[k] * g.H + iy[j]) * g.W + ix[i]) * C);
+          gx = fmaf(d, ex, gx); gy = fmaf(d, ey, gy); gz = fmaf(d, ez, gz);
+        }
+      }
+      continue;
+    }
+    // planes: (u -> fastest axis U, v -> slower axis V), as lp_taps
+    float u, v;
+    int U, V;
+    if (g.kind == LP_PLANE_XY) { u = x; v = y; U = g.W; V = g.H; }
+    else if (g.kind == LP_PLANE_XZ) { u = x; v = z; U = g.W; V = g.D; }
+    else { u = y; v = z; U = g.H; V = g.D; }
+    float wu[2], dwu[2], wv[2], dwv[2];
+    int iu[2], iv[2];
+    lp_axis_d(u, U, wu, dwu, iu);
+    lp_axis_d(v, V, wv, dwv, iv);
+    const long long bbase = g.base + (long long)b * U * V * C;
+    float gu = 0.f, gv = 0.f;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const int i = c & 1, j = c >> 1;
+      const float eu = dwu[i] * wv[j], ev = wu[i] * dwv[j];
+      if (eu != 0.f || ev != 0.f) {
+        const float d = dot(G.data + bbase + ((long long)iv[j] * U + iu[i]) * C);
+        gu = fmaf(d, eu, gu); gv = fmaf(d, ev, gv);
+      }
+    }
+    if (g.kind == LP_PLANE_XY) { gx += gu; gy += gv; }
+    else if (g.kind == LP_PLANE_XZ) { gx += gu; gz += gv; }
+    else { gy += gu; gz += gv; }
+  }
+}
+
+// Vector-Jacobian product of lp_contract at the pre-contraction point p: (gx, gy, gz), the gradient w.r.t. the
+// contracted point, becomes J_c(p)^T g.  Differentiated as autograd differentiates the MERF formula: a coordinate on the
+// max-norm n maps through (2 - 1/a) sign(v) -> 0.5 / a^2; the others through v / n -> 0.5 / n, plus -0.5 v / n^2 via n,
+// which reaches the coordinate(s) at the maximum (shared evenly between ties, like the gradient of a max).
+LP_DEVICE void lp_contract_vjp(float px, float py, float pz, float& gx, float& gy, float& gz) {
+  const float ax = fabsf(px), ay = fabsf(py), az = fabsf(pz);
+  const float n = fmaxf(fmaxf(ax, ay), az);
+  if (!(n > 1.f)) { gx *= 0.5f; gy *= 0.5f; gz *= 0.5f; return; }
+  float gn = 0.f;
+  auto one = [&](float v, float a, float& g) {
+    if (fabsf(a - n) <= 1e-8f) {
+      g = 0.5f * g / (a * a);
+    } else {
+      gn -= 0.5f * g * v / (n * n);
+      g = 0.5f * g / n;
+    }
+  };
+  one(px, ax, gx); one(py, ay, gy); one(pz, az, gz);
+  const float kx = ax == n ? 1.f : 0.f, ky = ay == n ? 1.f : 0.f, kz = az == n ? 1.f : 0.f;
+  const float share = gn / (kx + ky + kz);
+  gx += kx * (px < 0.f ? -share : share); gy += ky * (py < 0.f ? -share : share); gz += kz * (pz < 0.f ? -share : share);
 }
 
 // Nearest-neighbour lookup of a 1-channel voxel grid with zero padding and an additional

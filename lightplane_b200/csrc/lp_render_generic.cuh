@@ -41,6 +41,7 @@ struct LpBwdIo {
   const float* len; const float* feat; int feat_stride;
   const float* g_len; const float* g_nlt; const float* g_feat; int g_feat_stride;
   float* g_grid; float* g_cgrid; float* g_params; float* g_enc;
+  float* g_org; float* g_dir;  // [N,3] ray-geometry gradients (kernel instantiations with RAYG only; either may be NULL)
 };
 
 // Everything a renderer launch needs, built by lp_render_common() in lp_cabi.cu.
@@ -315,6 +316,26 @@ LP_DEVICE float* lp_mlp_backward(const LpMlp& Mlp, const float* P, float* dP, co
   return dy;
 }
 
+// Gradient w.r.t. the sample position of the lane's [C][lane] sampled-feature gradient tile (lp_lane_splat's adjoint
+// partner: the same taps, weighted by their weight gradients instead of their weights)
+LP_DEVICE void lp_lane_pos_grad(const LpGridSet& G, int b, float x, float y, float z, const float* tile, int lane,
+                                float& gx, float& gy, float& gz) {
+  const int C = G.C;
+  lp_pos_grad(G, b, x, y, z, [&](const float* row) {
+    float acc = 0.f;
+    for (int c = 0; c < C; c += 4) {
+      const float4 v = lp_ldg4(row + c);
+      acc = fmaf(v.x, tile[(c + 0) * LP_LS + lane], acc); acc = fmaf(v.y, tile[(c + 1) * LP_LS + lane], acc);
+      acc = fmaf(v.z, tile[(c + 2) * LP_LS + lane], acc); acc = fmaf(v.w, tile[(c + 3) * LP_LS + lane], acc);
+    }
+    return acc;
+  }, gx, gy, gz);
+}
+
+// RAYG: also the gradients w.r.t. the rays' origins and directions (io.g_org / io.g_dir, lp_render_backward_rays):
+// per sample j at p_j = o + t_j d, g_j = d L / d p_j from the taps' weight gradients (lp_pos_grad) and the contraction's
+// Jacobian; dL/do = sum_j g_j, dL/dd = sum_j t_j g_j.
+template <bool RAYG>
 __global__ void lp_render_bwd_generic_kernel(LpRays R, LpMarch M, LpDecoder D, LpActMap A, LpGridSet G,
                                              LpGridSet CG, LpGridSet SC, int use_scaffold,
                                              const float* __restrict__ params, int params_in_smem,
@@ -359,6 +380,7 @@ __global__ void lp_render_bwd_generic_kernel(LpRays R, LpMarch M, LpDecoder D, L
     total = fmaf(g, io.feat[(long long)rr * io.feat_stride + c], total);
   }
   float nlt = 0.f, T = 1.f, prefix = 0.f;
+  float gox = 0.f, goy = 0.f, goz = 0.f, gdx = 0.f, gdy = 0.f, gdz = 0.f;  // RAYG: dL/d origin, dL/d direction
 
   const int tot = M.S + M.S_inf;
   const int nc = D.color.n_layers, nt = D.trunk.n_layers;
@@ -367,6 +389,8 @@ __global__ void lp_render_bwd_generic_kernel(LpRays R, LpMarch M, LpDecoder D, L
     const float depth = lp_depth(step, s.near, s.far, M.S, M.S_inf, M.disparity_at_inf);
     const float delta = lp_delta(step, depth, s.near, s.far, M.S, M.S_inf, M.disparity_at_inf);
     float x = s.ox + depth * s.dx, y = s.oy + depth * s.dy, z = s.oz + depth * s.dz;
+    const float px = x, py = y, pz = z;
+    float gx = 0.f, gy = 0.f, gz = 0.f;  // RAYG: dL/d (grid-space sample point)
     if (M.contract) lp_contract(x, y, z);
     float occ = 1.f;
     if (use_scaffold) occ = lp_nearest(SC, s.b, x, y, z);
@@ -403,6 +427,7 @@ __global__ void lp_render_bwd_generic_kernel(LpRays R, LpMarch M, LpDecoder D, L
       for (int k = 0; k < D.C; ++k)
         if (!(xcs[k * LP_LS + lane] > 0.f)) d_xc[k * LP_LS + lane] = 0.f;
       lp_lane_splat(CG, io.g_cgrid, s.b, x, y, z, oob, d_xc, lane);
+      if (RAYG && oob != 0.f) lp_lane_pos_grad(CG, s.b, x, y, z, d_xc, lane, gx, gy, gz);
       for (int k = 0; k < D.C; ++k) gT[k * LP_LS + lane] = 0.f;
     } else {
       for (int k = 0; k < D.in_c; ++k) gT[k * LP_LS + lane] = d_xc[k * LP_LS + lane];
@@ -420,15 +445,26 @@ __global__ void lp_render_bwd_generic_kernel(LpRays R, LpMarch M, LpDecoder D, L
       // gA/gB/gT stay three distinct tiles, only their contents are consumed here
       float* d_x0 = lp_mlp_backward(D.trunk, P, dP, arena, arena + A.x0 * LP_LS, A.yt, gT, gA, lane);
       lp_lane_splat(G, io.g_grid, s.b, x, y, z, oob, d_x0, lane);
+      if (RAYG && oob != 0.f) lp_lane_pos_grad(G, s.b, x, y, z, d_x0, lane, gx, gy, gz);
     } else {
       const float* x0 = arena + A.x0 * LP_LS;  // relu-field: gate by relu(sampled) > 0
       for (int k = 0; k < D.C; ++k)
         if (!(x0[k * LP_LS + lane] > 0.f)) gT[k * LP_LS + lane] = 0.f;
       lp_lane_splat(G, io.g_grid, s.b, x, y, z, oob, gT, lane);
+      if (RAYG && oob != 0.f) lp_lane_pos_grad(G, s.b, x, y, z, gT, lane, gx, gy, gz);
+    }
+    if (RAYG) {
+      if (M.contract) lp_contract_vjp(px, py, pz, gx, gy, gz);
+      gox += gx; goy += gy; goz += gz;
+      gdx = fmaf(depth, gx, gdx); gdy = fmaf(depth, gy, gdy); gdz = fmaf(depth, gz, gdz);
     }
   }
   if (s.active)
     for (int k = 0; k < D.in_c; ++k) io.g_enc[(long long)ray * D.in_c + k] = genc[k * LP_LS + lane];
+  if (RAYG && s.active) {
+    if (io.g_org) { io.g_org[3 * ray] = gox; io.g_org[3 * ray + 1] = goy; io.g_org[3 * ray + 2] = goz; }
+    if (io.g_dir) { io.g_dir[3 * ray] = gdx; io.g_dir[3 * ray + 1] = gdy; io.g_dir[3 * ray + 2] = gdz; }
+  }
   __syncthreads();
   for (int i = threadIdx.x; i < D.n_params; i += blockDim.x) {
     const float v = dP[i];

@@ -187,8 +187,15 @@ LP_DEVICE void lp_ws_issue_encw_part(unsigned tmem, unsigned char* gs, int wi) {
 #define LP_WS_REGS_MEM(C) ((C) == 16 ? 88 : 128)
 #endif
 #define LP_WS_REGS_MLP(C) (256 - LP_WS_REGS_MEM(C))
+// With ray-geometry gradients (RAYG) the memory threads also hold the ray's six gradient sums and the re-gather's state
+#ifndef LP_WS_REGS_MEM_RAYG
+#define LP_WS_REGS_MEM_RAYG(C) ((C) == 16 ? 104 : 128)
+#endif
 
-template <int C, bool SCAF>
+// RAYG: also the gradients w.r.t. the rays' origins and directions (io.g_org / io.g_dir, either may be NULL).  Only the
+// memory role changes: when it consumes a slot's d_x0 it re-gathers the sample's tap rows and forms
+// g_j = sum_t <v_t, d_x0> grad w_t (lp_pos_grad) and J_c^T g_j; the owner thread of a ray sums them over the ray's samples.
+template <int C, bool SCAF, bool RAYG>
 __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMarch M, LpDecoder D, LpGridSet G, LpGridSet SC,
                                                                    const float* __restrict__ params, LpBwdIo io) {
   using I = Img<C>;
@@ -249,14 +256,16 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
   const int num_tiles = (R.n + GT - 1) / GT;
   const int tot = M.S + M.S_inf;
   const int tile0 = blockIdx.x * 2 + grp, tile_stride = gridDim.x * 2;
+  constexpr int REGS_MEM = RAYG ? LP_WS_REGS_MEM_RAYG(C) : LP_WS_REGS_MEM(C), REGS_MLP = 256 - REGS_MEM;
 
   if (!is_mlp) {
     // =================================================================================================================
     // memory group
     // =================================================================================================================
 #if LP_MEM_SINGLE_LOOP
-    if constexpr (LP_WS_REGS_MEM(C) < 128) LP_SETMAXNREG_DEC(LP_WS_REGS_MEM(C));
-    if constexpr (LP_WS_REGS_MEM(C) > 128) LP_SETMAXNREG_INC(LP_WS_REGS_MEM(C));
+    static_assert(!RAYG, "ray-geometry gradients are implemented in the unrolled memory role only");
+    if constexpr (REGS_MEM < 128) LP_SETMAXNREG_DEC(REGS_MEM);
+    if constexpr (REGS_MEM > 128) LP_SETMAXNREG_INC(REGS_MEM);
     int n_slot = 0, n_dw = 0, n_dx = 0;  // slots staged; dW GEMMs the decoder group has issued; d_x0 rows consumed
     for (int tile = tile0; tile < num_tiles; tile += tile_stride) {
       const Ray1 me = lp_load_ray1(R, lp_tile_ray(M, tile, s), G.g[0].B);
@@ -339,14 +348,15 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
       ++n_dw;  // the tile's tail: encoding product
     }
 #else
-    if constexpr (LP_WS_REGS_MEM(C) < 128) LP_SETMAXNREG_DEC(LP_WS_REGS_MEM(C));
-    if constexpr (LP_WS_REGS_MEM(C) > 128) LP_SETMAXNREG_INC(LP_WS_REGS_MEM(C));
+    if constexpr (REGS_MEM < 128) LP_SETMAXNREG_DEC(REGS_MEM);
+    if constexpr (REGS_MEM > 128) LP_SETMAXNREG_INC(REGS_MEM);
     int n_slot = 0, n_dw = 0, n_dx = 0;  // slots staged; dW GEMMs the decoder group has issued; d_x0 rows consumed
     for (int tile = tile0; tile < num_tiles; tile += tile_stride) {
       const Ray1 me = lp_load_ray1(R, lp_tile_ray(M, tile, s), G.g[0].B);
-      struct Pos { float x, y, z, oob; };
-      Pos prev = {0.f, 0.f, 0.f, 0.f};
+      struct Pos { float x, y, z, oob, t; };  // t: depth (RAYG)
+      Pos prev = {0.f, 0.f, 0.f, 0.f, 0.f};
       bool pend = false, any_empty = false;  // a full slot whose d_x0 is still to be scattered
+      float go[3] = {0.f, 0.f, 0.f}, gd[3] = {0.f, 0.f, 0.f};  // RAYG: dL/d origin, dL/d direction of the thread's ray
       // consume the d_x0 of the pending slot: read it, clear its accumulator columns, release them, scatter
       auto drain = [&](bool scatter) {
         float dxp[C];
@@ -361,6 +371,24 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
         if (scatter) {  // (warp-uniform) quad-transposed, footprint-merging reduction into the grid gradient
 #pragma unroll
           for (int c = 0; c < C; ++c) dxp[c] *= prev.oob;
+          if constexpr (RAYG) {
+            if (prev.oob != 0.f) {  // re-gather the taps (L2-resident), weighted by their weight gradients
+              float g[3] = {0.f, 0.f, 0.f};
+              lp_pos_grad(G, me.b, prev.x, prev.y, prev.z, [&](const float* row) {
+                float acc = 0.f;
+#pragma unroll
+                for (int k = 0; k < C / 4; ++k) {
+                  const float4 v = lp_ldg4(row + 4 * k);
+                  acc = fmaf(v.x, dxp[4 * k], acc); acc = fmaf(v.y, dxp[4 * k + 1], acc);
+                  acc = fmaf(v.z, dxp[4 * k + 2], acc); acc = fmaf(v.w, dxp[4 * k + 3], acc);
+                }
+                return acc;
+              }, g[0], g[1], g[2]);
+              if (M.contract) lp_contract_vjp(me.ox + prev.t * me.dx, me.oy + prev.t * me.dy, me.oz + prev.t * me.dz, g[0], g[1], g[2]);
+#pragma unroll
+              for (int k = 0; k < 3; ++k) { go[k] += g[k]; gd[k] = fmaf(prev.t, g[k], gd[k]); }
+            }
+          }
           lp_splat_quad<C, LP_BWD_TRI_SCATTER>(G, io.g_grid, me.b, prev.x, prev.y, prev.z, me.active && prev.oob != 0.f, dxp);
         }
       };
@@ -398,6 +426,7 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
         lp_depth_delta(sc, me.near, me.far, depth, delta);
         Pos cur;
         cur.x = me.ox + depth * me.dx; cur.y = me.oy + depth * me.dy; cur.z = me.oz + depth * me.dz;
+        if constexpr (RAYG) cur.t = depth;
         if (M.contract) lp_contract(cur.x, cur.y, cur.z);
         cur.oob = M.mask_oob ? lp_in_bounds(cur.x, cur.y, cur.z) : 1.f;
         const float occ = SCAF ? lp_nearest(SC, me.b, cur.x, cur.y, cur.z) : 1.f;
@@ -424,6 +453,10 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
       } else if (pend) {
         drain(true);
       }
+      if (RAYG && me.active) {  // each ray of the tile belongs to exactly one memory thread: plain stores
+        if (io.g_org) { io.g_org[3 * me.ray] = go[0]; io.g_org[3 * me.ray + 1] = go[1]; io.g_org[3 * me.ray + 2] = go[2]; }
+        if (io.g_dir) { io.g_dir[3 * me.ray] = gd[0]; io.g_dir[3 * me.ray + 1] = gd[1]; io.g_dir[3 * me.ray + 2] = gd[2]; }
+      }
       ++n_dw;  // the tile's tail: encoding product
     }
 #endif
@@ -431,8 +464,8 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
     // =================================================================================================================
     // decoder group
     // =================================================================================================================
-    if constexpr (LP_WS_REGS_MLP(C) > 128) LP_SETMAXNREG_INC(LP_WS_REGS_MLP(C));
-    if constexpr (LP_WS_REGS_MLP(C) < 128) LP_SETMAXNREG_DEC(LP_WS_REGS_MLP(C));
+    if constexpr (REGS_MLP > 128) LP_SETMAXNREG_INC(REGS_MLP);
+    if constexpr (REGS_MLP < 128) LP_SETMAXNREG_DEC(REGS_MLP);
     // one elected lane (elect.sync) of each of the group's four warps issues its share of every product
     const int wi = wig;
     const float* F = reinterpret_cast<const float*>(sm + I::F32);
@@ -810,7 +843,7 @@ __global__ void __launch_bounds__(512, 1) lp_render_bwd_ws_kernel(LpRays R, LpMa
   if (tid < 32) lp_tmem_dealloc512(tmem);
 }
 
-template <int C, bool SCAF>
+template <int C, bool SCAF, bool RAYG>
 static int lp_tc_render_backward_t(cudaStream_t st, const LpRenderArgs& a, const float* params, const LpBwdIo& io) {
   const int groups = 2;
   const int tiles = (a.R.n + GT - 1) / GT;
@@ -818,14 +851,19 @@ static int lp_tc_render_backward_t(cudaStream_t st, const LpRenderArgs& a, const
   const int max_blocks = lp_tc_num_sms();
   if (blocks > max_blocks) blocks = max_blocks;
   const size_t bytes = SImg<C>::GROUPS + (size_t)groups * SImg<C>::GROUP_BYTES;
-  if (LP_TC_SET_SMEM((lp_render_bwd_ws_kernel<C, SCAF>), bytes)) return LP_ERR_CUDA;
-  LP_LAUNCH((lp_render_bwd_ws_kernel<C, SCAF>), dim3(blocks), dim3(2 * groups * GT), bytes, st, a.R, a.M, a.D, a.G, a.SC, params, io);
+  if (LP_TC_SET_SMEM((lp_render_bwd_ws_kernel<C, SCAF, RAYG>), bytes)) return LP_ERR_CUDA;
+  LP_LAUNCH((lp_render_bwd_ws_kernel<C, SCAF, RAYG>), dim3(blocks), dim3(2 * groups * GT), bytes, st, a.R, a.M, a.D, a.G, a.SC, params, io);
   return LP_OK;
 }
-static inline int lp_tc_render_backward(cudaStream_t st, const LpRenderArgs& a, const float* params, const LpBwdIo& io) {
+template <bool RAYG>
+static int lp_tc_render_backward_r(cudaStream_t st, const LpRenderArgs& a, const float* params, const LpBwdIo& io) {
   if (a.use_scaffold)
-    return a.D.C == 16 ? lp_tc_render_backward_t<16, true>(st, a, params, io) : lp_tc_render_backward_t<32, true>(st, a, params, io);
-  return a.D.C == 16 ? lp_tc_render_backward_t<16, false>(st, a, params, io) : lp_tc_render_backward_t<32, false>(st, a, params, io);
+    return a.D.C == 16 ? lp_tc_render_backward_t<16, true, RAYG>(st, a, params, io) : lp_tc_render_backward_t<32, true, RAYG>(st, a, params, io);
+  return a.D.C == 16 ? lp_tc_render_backward_t<16, false, RAYG>(st, a, params, io) : lp_tc_render_backward_t<32, false, RAYG>(st, a, params, io);
+}
+// rayg: the launch also writes io.g_org / io.g_dir
+static inline int lp_tc_render_backward(cudaStream_t st, const LpRenderArgs& a, const float* params, const LpBwdIo& io, bool rayg) {
+  return rayg ? lp_tc_render_backward_r<true>(st, a, params, io) : lp_tc_render_backward_r<false>(st, a, params, io);
 }
 
 }  // namespace lptc

@@ -5,13 +5,18 @@ keeps its signature and return values; `LightplaneFunction` (:296-756) is the
 `torch.autograd.Function` whose forward / backward now call `lp_render_forward` /
 `lp_render_backward` of `include/lightplane_b200.h` instead of launching Triton kernels.
 
+Extension: gradients w.r.t. the ray origins and directions (`lp_render_backward_rays`) when either
+requires grad -- e.g. for refining camera poses from a photometric loss; the reference returns none.
+
 Differences a caller can observe, all deliberate (DESIGN.md "Boundary"):
   * no host synchronisation: shapes are validated from metadata only; `grid_idx` range is
     clamped in the kernel (set `lightplane_renderer.VALIDATE_INPUTS = True` for the
     reference's device-side asserts, lightplane_renderer.py:464-467);
   * rays are not padded to a multiple of 16 and the padded colour channels are neither computed
     nor stored (the reference crops them right after the launch, :284-291);
-  * `regenerate_code`, `triton_block_size`, `triton_num_warps` are accepted and ignored.
+  * `regenerate_code`, `triton_block_size`, `triton_num_warps` are accepted and ignored;
+  * `rays.origins` / `rays.directions` that require grad receive their gradient (the reference's
+    backward returns None for them); `near` / `far` still get none.
 """
 
 from __future__ import annotations
@@ -147,7 +152,11 @@ class LightplaneFunction(torch.autograd.Function):
     """autograd binding of the fused ray-march kernels.
 
     Differentiable inputs: flat feature grid, mlp_params, ray encoding, flat colour grid
-    (as in the reference, lightplane_renderer.py:724-756; no gradient w.r.t. ray geometry).
+    (as in the reference, lightplane_renderer.py:724-756) and, as an extension, the ray directions
+    and origins: when either requires grad the backward calls `lp_render_backward_rays`, which adds
+    dL/d origin = sum_j J_c(p_j)^T g_j and dL/d direction = sum_j t_j J_c(p_j)^T g_j over the samples
+    p_j = o + t_j d (g_j: the gradient w.r.t. the grid-space sample point; J_c: the contraction's
+    Jacobian).  Without it the backward is exactly `lp_render_backward`.
     Only per-ray tensors are saved for backward (the forward outputs `ray_length`, `features`
     and the inputs) -- the backward kernel recomputes every per-sample quantity.
     """
@@ -287,6 +296,7 @@ class LightplaneFunction(torch.autograd.Function):
             ray_length, features, feature_grid_c, mlp_params_c, enc_c, color_c, dirs_c, orig_c,
             gidx_c, near_c, far_c, scaf_c,
         )
+        ctx.ray_dtypes = (directions.dtype, origins.dtype)
         ctx.lp = (cfg, spec, grid_sizes, color_grid_sizes,
                   None if scaffold is None else list(scaffold.shape) + [1], color_chn)
         return ray_length, nlt, features
@@ -319,22 +329,32 @@ class LightplaneFunction(torch.autograd.Function):
         color_s = _cabi.make_grid_list(color_grid, color_grid_sizes) if color_grid is not None else None
         scaf_s = _cabi.make_grid_list(scaf, [scaf_size]) if scaf is not None else None
 
+        # inputs 6 / 7 of forward(): directions, origins
+        want_dir, want_org = ctx.needs_input_grad[6], ctx.needs_input_grad[7]
+        grad_dir = torch.empty_like(dirs) if want_dir else None
+        grad_org = torch.empty_like(orig) if want_org else None
+        args = (_cabi.stream_ptr(device),
+                _byref(cfg), _byref(spec), _byref(rays_s), _byref(grid_s),
+                _byref(color_s), _byref(scaf_s),
+                mlp_params.data_ptr(), ray_length.data_ptr(), features.data_ptr(), color_chn,
+                g_len.data_ptr(), g_nlt.data_ptr(), g_feat.data_ptr(), color_chn,
+                grad_grid.data_ptr(), _cabi.ptr(grad_color), grad_mlp.data_ptr(),
+                grad_enc.data_ptr())
+        entry = "lp_render_backward_rays" if (want_dir or want_org) else "lp_render_backward"
+        if entry == "lp_render_backward_rays":
+            args += (_cabi.ptr(grad_org), _cabi.ptr(grad_dir))
         if num_rays > 0:
             with torch.cuda.device(device):
-                st = _cabi.call(lib, "lp_render_backward",
-                    _cabi.stream_ptr(device),
-                    _byref(cfg), _byref(spec), _byref(rays_s), _byref(grid_s),
-                    _byref(color_s), _byref(scaf_s),
-                    mlp_params.data_ptr(), ray_length.data_ptr(), features.data_ptr(), color_chn,
-                    g_len.data_ptr(), g_nlt.data_ptr(), g_feat.data_ptr(), color_chn,
-                    grad_grid.data_ptr(), _cabi.ptr(grad_color), grad_mlp.data_ptr(),
-                    grad_enc.data_ptr(),
-                )
-            _cabi.check(lib, st, "lp_render_backward")
+                st = _cabi.call(lib, entry, *args)
+            _cabi.check(lib, st, entry)
         else:
             grad_enc.zero_()
+        if grad_dir is not None:
+            grad_dir = grad_dir.to(ctx.ray_dtypes[0])
+        if grad_org is not None:
+            grad_org = grad_org.to(ctx.ray_dtypes[1])
 
-        return (grad_grid, grad_mlp, grad_enc, grad_color) + (None,) * 18
+        return (grad_grid, grad_mlp, grad_enc, grad_color, None, None, grad_dir, grad_org) + (None,) * 14
 
 
 def _byref(s):
